@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our CUDA path (default N=1)
     python bench.py --impl reference --steps K --warmup W     # the reference's own CPU superagg on the host cores
+    python bench.py --steps K --warmup W --dump-outputs DIR   # also write the last timed step's grid to DIR/count.npy
 
 One "step" = one pass of the hot path over the whole synthetic batch (rows_per_gpu rows on every rank):
 reset grid -> fused binby kernel -> (N>1) NCCL all-reduce of the 1027^2 int64 grid -> D2H of the grid.
@@ -43,7 +44,22 @@ def parse():
     ap.add_argument("--no-overlap", action="store_true", help="serialise every step's all-reduce + D2H behind its kernels (default: they run on a second stream under the next step)")
     ap.add_argument("--no-also", action="store_true", help="skip the other BASELINE.json configs (sum, 3-D mean+std, groupby)")
     ap.add_argument("--also-sample", type=float, default=1e8, help="rows of the parity sample of each `also` config against oracle/_ref")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the count grid of the last timed step to DIR/count.npy (float64, the shape "
+                                                          "get_result() returns), to compare two builds on the same seeded inputs")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the CUDA path computed: use it with --impl b200")
+    return args
+
+
+def dump_outputs(path, arrays):
+    """one <name>.npy per array, as float64 (exact for counts below 2^53)"""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -528,6 +544,8 @@ def run_b200(args):
     for hg in host_grids[: min(2, nstep[0])]:
         counted = int(hg.sum().item())
         assert counted == rows * world, f"row conservation failed: grid holds {counted}, expected {rows * world}"
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"count": host_grids[(nstep[0] - 1) % 2].numpy().reshape(grid.shapes, order="F")})
 
     value = rows * world * args.steps / (total_ms * 1e-3)
     # count(*) on a 1027^2 grid takes the ring-partition path from 2^22 rows: 2 kernels (+ 2 memsets) per batch of <= 2^30 rows

@@ -17,13 +17,3 @@ def oracle():
     from oracle import oracle as O
     O.lib()
     return O
-
-
-@pytest.fixture(scope="session")
-def ref():
-    """The compiled, unmodified reference (oracle/_ref); skips when it was not built."""
-    from oracle import ref_driver
-    if not ref_driver.available():
-        pytest.skip("oracle/_ref not built (make -C oracle ref)")
-    ref_driver.modules()
-    return ref_driver

@@ -76,6 +76,29 @@ def load_strings():
     return cases
 
 
+PINNING_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "pinning_golden.npz")
+
+
+def load_pinning():
+    """tests/golden/pinning_golden.npz (tests/golden/make_golden_pinning.py): name -> dict of arrays"""
+    z = np.load(PINNING_PATH, allow_pickle=False)
+    cases = {}
+    for key in z.files:
+        name, field = key.split("/", 1)
+        cases.setdefault(name, {})[field] = z[key]
+    return cases
+
+
+def pinned_results(c):
+    """the a<k>_result (+ a<k>_result_mask) arrays of a pinning case -> the reference's result list (numpy.ma where masked)"""
+    out = []
+    while f"a{len(out)}_result" in c:
+        k = len(out)
+        r = c[f"a{k}_result"]
+        out.append(np.ma.array(r, mask=c[f"a{k}_result_mask"]) if f"a{k}_result_mask" in c else r)
+    return out
+
+
 AGGLIST_PATH = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "agglist_golden.npz")
 
 

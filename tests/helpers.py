@@ -172,3 +172,65 @@ def random_case(rng, n, allow_first=True, float_sum_ok=True):
         else:
             aggs.append(O.agg(op, data, mask))
     return binners, aggs
+
+
+# ---- cases pinned to the compiled reference in tests/golden/pinning_golden.npz (tests/golden/make_golden_pinning.py) -----------
+def random_binby_case(seed):
+    rng = np.random.default_rng(1000 + seed)
+    n = int(rng.integers(1, 5000))
+    binners, aggs = random_case(rng, n)
+    return binners, aggs, n
+
+
+def first_mask_quirk_case():
+    """first / last past 1024 rows with a data mask: AggFirst indexes its mask inside the 1024-row block without the block offset
+    (src/agg_first.cpp:131)"""
+    from oracle import oracle as O
+    rng = np.random.default_rng(77)
+    n = 3000
+    x = rng.uniform(0, 4, n)
+    v = rng.normal(0, 1, n)
+    o = rng.integers(0, 100, n).astype("i8")
+    m = (rng.random(n) < 0.6).astype("u1")
+    return [O.scalar(x, 0, 4, 4)], [O.agg("first", v, m, order=o), O.agg("last", v, m, order=o)], n
+
+
+CHUNK_LOOP_THREADS = (1, 4)
+CHUNK_LOOP_CHUNK = 50_000
+
+
+def chunk_loop_case():
+    from oracle import oracle as O
+    rng = np.random.default_rng(5)
+    n = 300_000
+    x = rng.normal(0, 1, n).astype("f4")
+    y = rng.normal(0, 1, n).astype("f4")
+    return [O.scalar(x, -3, 3, 64), O.scalar(y, -3, 3, 64)], [O.agg("count")], n
+
+
+MINMAX_RANDOM_DTYPES = ("f8", "f4", "i8", "i4", "i2", "i1", "u8", "u4", "u2", "u1", "?", ">f8", ">i4", ">u2")
+
+
+def minmax_random_columns(seed):
+    """(dtype, column) pairs for df.minmax: every dtype of MINMAX_RANDOM_DTYPES plain, then half masked"""
+    rng = np.random.default_rng(4000 + seed)
+    n = int(rng.integers(1, 20000))
+    out = []
+    for dt in MINMAX_RANDOM_DTYPES:
+        d = np.dtype(dt)
+        if d.kind == "f":
+            v = (rng.standard_normal(n) * 10.0 ** int(rng.integers(-3, 6))).astype(d)
+            v[rng.random(n) < 0.2] = np.nan
+        elif d.kind == "b":
+            v = rng.integers(0, 2, n).astype(d)
+        else:
+            info = np.iinfo(d)
+            v = rng.integers(info.min, info.max, n, dtype=np.int64 if d.kind == "i" else np.uint64, endpoint=True).astype(d)
+        out += [(dt, v), (dt, np.ma.array(v, mask=rng.random(n) < 0.5))]
+    return out
+
+
+def grid_layout_binners(superagg):
+    """a scalar, an ordinal and an ordinal-with-other binner of `superagg` (the reference's module or the mirror)"""
+    return [superagg.BinnerScalar_float64(1, "x", 0, 1, 5), superagg.BinnerOrdinal_int32(1, "y", 4, 0, False, False),
+            superagg.BinnerOrdinal_int8(1, "z", 3, 0, True, False)]

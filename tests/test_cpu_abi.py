@@ -7,6 +7,9 @@ import re
 import numpy as np
 import pytest
 
+import golden_util
+from helpers import grid_layout_binners
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -42,17 +45,17 @@ def test_hash64_known_answers():
     assert superutils.hash(2) == 15839785061582574730
 
 
-def test_mirror_class_names_match_reference(ref):
-    """every numeric Binner*/Agg* name of the compiled reference module resolves in the mirror"""
-    superagg, superutils = ref.modules()
+def test_mirror_class_names_match_reference():
+    """every numeric Binner*/Agg* name of the compiled reference module resolves in the mirror (names stored by
+    tests/golden/make_golden_pinning.py)"""
     from vaex_b200 import superagg as mine, superutils as myutils
-    want = [n for n in dir(superagg) if n.startswith(("BinnerScalar_", "BinnerOrdinal_", "AggCount_", "AggSum_", "AggSumMoment_", "AggMin_", "AggMax_", "AggFirst_", "AggNUnique_"))
-            and not n.endswith(("_string", "_object"))]
+    names = golden_util.load_pinning()["names"]
+    want = [str(n) for n in names["superagg"]]
     assert len(want) > 300
     missing = [n for n in want if not hasattr(mine, n)]
     assert not missing, missing[:10]
     assert hasattr(mine, "Grid")
-    sets = [n for n in dir(superutils) if n.startswith("ordered_set_") and n not in ("ordered_set_string", "ordered_set_object")]
+    sets = [str(n) for n in names["ordered_sets"]]
     assert len(sets) == 11
     assert not [n for n in sets if not hasattr(myutils, n)]
 
@@ -79,14 +82,14 @@ def test_no_cpu_fallback():
         superutils.ordered_set_int64(1)
 
 
-def test_grid_layout_matches_reference(ref):
-    superagg, _ = ref.modules()
+def test_grid_layout_matches_reference():
+    """the mirror's Grid over grid_layout_binners has the shapes, strides and length the compiled reference's Grid has"""
     from vaex_b200 import superagg as mine
-    rb = [superagg.BinnerScalar_float64(1, "x", 0, 1, 5), superagg.BinnerOrdinal_int32(1, "y", 4, 0, False, False), superagg.BinnerOrdinal_int8(1, "z", 3, 0, True, False)]
-    mb = [mine.BinnerScalar_float64(1, "x", 0, 1, 5), mine.BinnerOrdinal_int32(1, "y", 4, 0, False, False), mine.BinnerOrdinal_int8(1, "z", 3, 0, True, False)]
-    rg, mg = superagg.Grid(rb), mine.Grid(mb)
-    assert list(rg.shapes) == mg.shapes and list(rg.strides) == mg.strides and len(rg) == len(mg)
-    assert [len(b) for b in rb] == [len(b) for b in mb]
+    want = golden_util.load_pinning()["grid_layout"]
+    mb = grid_layout_binners(mine)
+    mg = mine.Grid(mb)
+    assert want["shapes"].tolist() == mg.shapes and want["strides"].tolist() == mg.strides and int(want["length"]) == len(mg)
+    assert want["binner_lengths"].tolist() == [len(b) for b in mb]
 
 
 def test_binner_errors_match_reference():

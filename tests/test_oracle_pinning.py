@@ -1,13 +1,13 @@
-"""Pin the oracle (oracle/binstats_oracle.c) — CPU only.
-
- 1. against the golden vectors generated from the compiled, unmodified reference (tests/golden/, always available);
- 2. against the compiled reference itself (oracle/_ref) on fresh random cases when it is present in this container.
+"""Pin the oracle (oracle/binstats_oracle.c) — CPU only — against the golden vectors generated from the compiled, unmodified
+reference (tests/golden/): known-answer and fixed cases stored with their inputs, and random / quirk cases whose inputs
+tests/helpers.py rebuilds from a seed (tests/golden/pinning_golden.npz).
 The oracle is the checker of every GPU parity test, so it has to be right first."""
 import numpy as np
 import pytest
 
 import golden_util
-from helpers import random_case, same
+from helpers import (CHUNK_LOOP_THREADS, MINMAX_RANDOM_DTYPES, chunk_loop_case, first_mask_quirk_case, minmax_random_columns, random_binby_case,
+                     same)
 
 GOLD = golden_util.load()
 BINBY = sorted(k for k in GOLD if not k.startswith(("set_", "hash64")))
@@ -48,44 +48,39 @@ def test_hash64_golden(oracle):
     assert oracle.hash64(1) == 6238072747940578789  # SURVEY.md 8c pin
 
 
+# ---- the compiled reference's answers on the cases of tests/helpers.py (tests/golden/pinning_golden.npz) -------------------------
+PINNED = golden_util.load_pinning()
+
+
 @pytest.mark.parametrize("seed", range(12))
-def test_oracle_matches_compiled_reference_random(seed, oracle, ref):
-    rng = np.random.default_rng(1000 + seed)
-    n = int(rng.integers(1, 5000))
-    binners, aggs = random_case(rng, n)
-    want = ref.binby(binners, aggs, n)
+def test_oracle_matches_compiled_reference_random(seed, oracle):
+    binners, aggs, n = random_binby_case(seed)
+    want = golden_util.pinned_results(PINNED[f"random_{seed}"])
     got = oracle.binby(binners, aggs, n)
+    assert len(want) == len(aggs)
     for a, w, g in zip(aggs, want, got):
-        assert same(np.asarray(w) if not np.ma.isMaskedArray(w) else w, g), (a["op"], None if a["data"] is None else a["data"].dtype)
+        assert same(w, g), (a["op"], None if a["data"] is None else a["data"].dtype)
 
 
-def test_oracle_first_mask_quirk_matches_reference(oracle, ref):
+def test_oracle_first_mask_quirk_matches_reference(oracle):
     """AggFirst indexes its mask inside the 1024-row block without the block offset (src/agg_first.cpp:131);
     the oracle restates that, so both agree even past 1024 rows."""
-    rng = np.random.default_rng(77)
-    n = 3000
-    x = rng.uniform(0, 4, n)
-    v = rng.normal(0, 1, n)
-    o = rng.integers(0, 100, n).astype("i8")
-    m = (rng.random(n) < 0.6).astype("u1")
-    b = [oracle.scalar(x, 0, 4, 4)]
-    a = [oracle.agg("first", v, m, order=o), oracle.agg("last", v, m, order=o)]
-    for w, g in zip(ref.binby(b, a, n), oracle.binby(b, a, n)):
+    b, a, n = first_mask_quirk_case()
+    want = golden_util.pinned_results(PINNED["first_mask_quirk"])
+    assert len(want) == 2
+    for w, g in zip(want, oracle.binby(b, a, n)):
         assert same(w, g)
 
 
-@pytest.mark.parametrize("nthreads", [1, 4])
-def test_reference_chunk_loop_is_thread_invariant_for_counts(nthreads, oracle, ref):
-    """the restated executor loop (1M-row chunks, per-thread grids folded in get_result) gives the same exact counts"""
-    rng = np.random.default_rng(5)
-    n = 300_000
-    x = rng.normal(0, 1, n).astype("f4")
-    y = rng.normal(0, 1, n).astype("f4")
-    b = [oracle.scalar(x, -3, 3, 64), oracle.scalar(y, -3, 3, 64)]
-    a = [oracle.agg("count")]
+@pytest.mark.parametrize("nthreads", CHUNK_LOOP_THREADS)
+def test_reference_chunk_loop_is_thread_invariant_for_counts(nthreads, oracle):
+    """the reference's executor loop (50k-row chunks over `nthreads` threads, per-thread grids folded in get_result) gives the
+    counts of one sequential pass"""
+    b, a, n = chunk_loop_case()
     want = oracle.binby(b, a, n)[0]
-    got = ref.RefBinby(b, a, nthreads).run(n, chunk=50_000)[0]
-    assert np.array_equal(want, np.asarray(got))
+    got = golden_util.pinned_results(PINNED[f"chunk_loop_{nthreads}"])[0]
+    assert int(got.sum()) == n
+    assert np.array_equal(want, got)
 
 
 # ---- limits pre-pass (df.minmax): SURVEY.md section 8f row 1 ------------------------------------------------------------------
@@ -111,21 +106,12 @@ def test_minmax_float_cast_quirk_is_in_the_golden_vectors():
 
 
 @pytest.mark.parametrize("seed", range(6))
-def test_oracle_minmax_matches_compiled_reference_random(seed, oracle, ref):
-    rng = np.random.default_rng(4000 + seed)
-    n = int(rng.integers(1, 20000))
-    for dt in ("f8", "f4", "i8", "i4", "i2", "i1", "u8", "u4", "u2", "u1", "?", ">f8", ">i4", ">u2"):
-        d = np.dtype(dt)
-        if d.kind == "f":
-            v = (rng.standard_normal(n) * 10.0 ** int(rng.integers(-3, 6))).astype(d)
-            v[rng.random(n) < 0.2] = np.nan
-        elif d.kind == "b":
-            v = rng.integers(0, 2, n).astype(d)
-        else:
-            info = np.iinfo(d)
-            v = rng.integers(info.min, info.max, n, dtype=np.int64 if d.kind == "i" else np.uint64, endpoint=True).astype(d)
-        for col in (v, np.ma.array(v, mask=rng.random(n) < 0.5)):
-            assert np.array_equal(oracle.minmax(col, raw=True), ref.minmax(col, raw=True), equal_nan=True), dt
+def test_oracle_minmax_matches_compiled_reference_random(seed, oracle):
+    cols = minmax_random_columns(seed)
+    want = PINNED[f"minmax_{seed}"]["raw"]
+    assert len(want) == len(cols) == 2 * len(MINMAX_RANDOM_DTYPES)
+    for (dt, col), w in zip(cols, want):
+        assert np.array_equal(oracle.minmax(col, raw=True), w, equal_nan=True), dt
 
 
 # ---- string key sets (SURVEY.md section 8f row 3) ----------------------------------------------------------------------------------

@@ -77,7 +77,14 @@ typedef enum {
                         bit 1 = dropnan.  b200_agg_input: `mask` = validity (1 = value present, 0 = null row: the reference's
                         data mask), `order` = selection mask (uint8, 1 = the row takes part: set_selection_mask); both nullable */,
     B200_AGG_LIST /* AggList_<T>(grid, grids, threads, dropnan, dropnull) (src/agg_list.cpp:5-127): `moment` bit 0 = dropnan, bit 1 =
-                     dropnull; read with b200_agg_list_finish / b200_agg_list_read, not b200_agg_read */
+                     dropnull; read with b200_agg_list_finish / b200_agg_list_read, not b200_agg_read */,
+    B200_AGG_LIST_STRING /* AggList_string_int64(grid, grids, threads, dropnan, dropnull) (src/agg_list.cpp:122-222): per cell the
+                            strings in arrival order, a null string as a null element where it arrived (unless dropnull).  `moment` bit 1
+                            = dropnull; bit 0 (dropnan) is accepted and has no effect, like in the reference; `dtype` is B200_U8.
+                            b200_agg_input: `data` = int64 string offsets[nrows + 1] (arrow large_string; offsets[0] may be > 0),
+                            `order` = the bytes they index (NULL only when no row has a byte), `mask` = null mask of the strings
+                            (1 = null; nullable).  There is no data mask: the reference never reads it.  Read with
+                            b200_agg_list_string_finish / b200_agg_list_string_read.  Fewer than 2^32 rows per aggregator. */
 } b200_agg_op;
 
 /* where the column pointers of a call live.  MIXED: every pointer is classified on its own (cudaPointerGetAttributes);
@@ -169,6 +176,12 @@ int b200_agg_merge(b200_agg *agg, b200_agg *const *others, int nothers);
  * offsets[cells + 1] and `total` values of the aggregator's dtype.  merge() is a no-op like the reference's (:46). */
 int b200_agg_list_finish(b200_agg *agg, int64_t *total_out);
 int b200_agg_list_read(b200_agg *agg, int64_t *offsets_out, void *values_out);
+/* AggListString::get_result (src/agg_list.cpp:141-182).  finish: sorts the appended records (stable, by cell) and builds the result on
+ * the device; nelem = elements over all cells, nbytes = their bytes.  read: one D2H per buffer, any may be NULL: list_offsets =
+ * int64[cells + 1], str_offsets = int64[nelem + 1] (arrow large_string offsets, starting at 0), bytes[nbytes], nulls[nelem] (1 = null
+ * element, which has no bytes).  merge() is a no-op like the reference's (:140). */
+int b200_agg_list_string_finish(b200_agg *agg, int64_t *nelem_out, int64_t *nbytes_out);
+int b200_agg_list_string_read(b200_agg *agg, int64_t *list_offsets, int64_t *str_offsets, uint8_t *bytes, uint8_t *nulls);
 /* load a full grid (result dtype, `cells` long) — TaskPartAggregation initial_values (vaex/cpu.py:654-658) */
 int b200_agg_write(b200_agg *agg, const void *values);
 

@@ -24,7 +24,7 @@ DTYPES = ["float64", "float32", "int64", "int32", "int16", "int8", "uint64", "ui
 DTYPE_CODE = {n: i for i, n in enumerate(DTYPES)}
 F64, F32, I64, I32, I16, I8, U64, U32, U16, U8, BOOL = range(11)
 BINNER_SCALAR, BINNER_ORDINAL, BINNER_HASH = 0, 1, 2
-AGG_COUNT, AGG_SUM, AGG_SUM_MOMENT, AGG_MIN, AGG_MAX, AGG_FIRST, AGG_LAST, AGG_NUNIQUE, AGG_LIST = range(9)
+AGG_COUNT, AGG_SUM, AGG_SUM_MOMENT, AGG_MIN, AGG_MAX, AGG_FIRST, AGG_LAST, AGG_NUNIQUE, AGG_LIST, AGG_LIST_STRING = range(10)
 MEM_HOST, MEM_DEVICE, MEM_MIXED = 0, 1, 2
 FLAG_ASYNC_HOST = 1
 ERR_NODATA = -3
@@ -120,6 +120,8 @@ def lib():
             "b200_agg_merge": (i32, [vp, P(vp), i32]),
             "b200_agg_list_finish": (i32, [vp, P(i64)]),
             "b200_agg_list_read": (i32, [vp, vp, vp]),
+            "b200_agg_list_string_finish": (i32, [vp, P(i64), P(i64)]),
+            "b200_agg_list_string_read": (i32, [vp, vp, vp, vp, vp]),
             "b200_agg_write": (i32, [vp, vp]),
             "b200_bin": (i32, [vp, i32, P(Binner), i32, P(AggInput), i32, i64, i64, i32, u32]),
             "b200_eval": (i32, [vp, i32, P(ExprOp), i32, P(ExprInput), i32, P(vp), i32, i64, i32, i32, vp]),

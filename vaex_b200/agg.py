@@ -4,8 +4,8 @@ Reference: packages/vaex-core/vaex/agg.py:221-335 (AggregatorDescriptorBasic: en
 grid-count heuristic and memory accounting, get_result edge slicing), :386-523 (mean / var / std / skew / kurtosis as
 combinations of primitive grids + ``finish``), :525-606 (count, sum, mean, min, max, first, last, std, var, ...).
 The primitive aggregations run on the GPU (vaex_b200.superagg); ``finish`` is O(cells) numpy like in the reference.
-nunique (vaex/agg.py:338-369, 600-612) runs on the device too.  Out of scope here (SURVEY.md 8f): list, describe, string/object
-columns.
+nunique (vaex/agg.py:338-369, 600-612) and list, on numeric and string columns, run on the device too.  Out of scope here
+(SURVEY.md 8f): describe, object columns.
 """
 import operator
 from functools import reduce
@@ -31,8 +31,10 @@ def _upcast(dtype):
 def find_type_from_dtype(namespace, prefix, dtype, *others):
     """vaex.utils.find_type_from_dtype (vaex/utils.py:754-791): ``prefix + dtype [+ '_' + dtype2] [+ '_non_native']``."""
     dtype = np.dtype(dtype)
-    if dtype.kind in "OU":  # string columns: the reference's classes carry the suffix "string"
+    if dtype.kind in "OU":  # string columns: the reference's classes carry the suffix "string" (+ "_<dtype2>", AggList_string_int64)
         name = prefix + "string"
+        for o in others:
+            name += "_" + np.dtype(o).newbyteorder("=").name
         if not hasattr(namespace, name):
             raise ValueError(f"Could not find a class ({name}), seems strings are not supported.")
         return getattr(namespace, name)

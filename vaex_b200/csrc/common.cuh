@@ -139,6 +139,16 @@ struct b200_agg {
     unsigned *list_counts = nullptr;       // after finish: exclusive offsets per cell (+ the total)
     uint64_t list_n = 0, list_cap = 0, list_total = 0;
     bool list_sorted = false;
+    // LIST_STRING (list.cu): the records above with key = cell and payload = arrival index (bit 63: null string); every call's bytes
+    // are appended to one device pool, record r's bytes start at str_start[r] (its length: str_start[r + 1] - str_start[r])
+    unsigned char *str_pool = nullptr;
+    uint64_t str_pool_n = 0, str_pool_cap = 0;
+    unsigned long long *str_start = nullptr; // list_cap + 1 entries
+    // after finish: int64 string offsets[list_total + 1], the gathered bytes, one null flag per element
+    long long *str_off = nullptr;
+    unsigned char *str_bytes = nullptr, *str_nulls = nullptr;
+    uint64_t str_nbytes = 0, str_elem_cap = 0, str_bytes_cap = 0;
+    bool str_ready = false; // the buffers hold the result of the last finish (cleared by a new row or a reset)
 };
 
 namespace b200 {
